@@ -19,8 +19,13 @@ per rank, at every N), `offline_bf16_256` (configs[2]), `enrollment_1024` (confi
 `--impl reference` times the reference's own CPU path (the reference modules when the checkout is
 present, else the oracle port) on the host cores with the same workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--chunks-per-call C] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--chunks-per-call C] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+
+`--dump-outputs DIR` writes what the last timed step of each arm handed back to its caller (rank 0), float32:
+y.npy (the separated clip of the device-resident arm), state.*.npy (its streaming state after the clip, in the
+reference's layout, SepState.to_reference) and y_e2e.npy (the clip of the host-buffer arm).  Inputs and weights
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -232,6 +237,33 @@ def measure_enrollment(dev, nb=1024, n=80000):
     return ms
 
 
+DUMP_BYTES = 60e6       # --dump-outputs thins above this; the per-row rounding of the thinning keeps it under 64 MB
+
+
+def step_outputs(net, y, st):
+    """Host copies of what a device-resident step hands its caller: the separated clip `y` and the streaming state `st`,
+    the state converted to the reference's layout on a host copy (no device memory is allocated)."""
+    from lookoncetohear_b200.net import SepState
+    ref = SepState(st.buf.cpu(), st.batch, st.n_blocks, *net._state_layout()).to_reference()
+    out = {"y": y.cpu()}
+    out.update({f"state.{k}": ref[k] for k in ("conv_buf", "deconv_buf", "istft_buf")})
+    for b, bufs in ref["gridnet_bufs"].items():
+        out.update({f"state.{b}.{k}": v for k, v in bufs.items()})
+    return out
+
+
+def write_outputs(out_dir, arrays):
+    """out_dir/<name>.npy in float32 for every array.  Should they come to more than DUMP_BYTES (a long --clip-hops),
+    every array keeps every k-th element of its last axis, the same k for all."""
+    import math
+
+    import numpy as np
+    k = max(1, math.ceil(sum(4 * t.numel() for t in arrays.values()) / DUMP_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t[..., ::k].float().numpy())
+
+
 def run_reference(args, rank, world):
     if rank != 0:
         return
@@ -277,6 +309,8 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the latency / buffered-throughput extras")
     ap.add_argument("--clip-hops", type=int, default=0,
                     help="profiling aid: shorten the clip to this many hops (the default, 0, is the 4 s = 500-hop clip)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32), see the module docstring")
     args = ap.parse_args()
 
     global CLIP_SAMPLES, FRAMES
@@ -359,6 +393,9 @@ def main():
     n_launched = ctypes.c_int64()
     _cabi.check(L.l2h_sep_launch_count(net._engine(), ctypes.byref(n_launched), 0))
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        dump = step_outputs(net, y_dev, net._last_stream_state)    # stream_dev keeps the state of its last call
     # ---- end-to-end arm (host buffers, H2D/D2H inside) -----------------------------------------------
     for _ in range(min(args.warmup, 2)):
         step_host()
@@ -373,6 +410,9 @@ def main():
     e2e_wall = time.perf_counter() - t0
     e2e_ms = max(e0.elapsed_time(e1), 1e3 * e2e_wall)          # the call ends with a stream sync; take the larger
     clocks = sampler.result()
+    if dump is not None:
+        dump["y_e2e"] = y_host
+        write_outputs(args.dump_outputs, dump)
 
     # ---- configs[4] per-GPU shape on EVERY rank: 256 streams per rank, one hop per step, max-over-ranks time ----
     bs_ms, bs_gb, bs_err = 0.0, 0.0, None

@@ -3,9 +3,9 @@
 CPU restatement of the reference's hot path, written from the formulas (SURVEY.md Appendix
 A / B), independent of the reference's module graph.  It travels to the GPU box (where
 /root/reference does not exist) and is the checker the ``-m gpu`` parity tests, ``smoke()``
-and ``bench.py``'s cpu_baseline use.  It is itself pinned against the reference's own code run
-in the build container (tests/test_oracle.py, needs /root/reference) and against the committed
-fixtures in tests/golden/ (generated by tests/golden/make_golden.py from the reference).
+and ``bench.py``'s cpu_baseline use.  It is itself pinned against results of the reference's own
+code (tests/test_oracle.py), recorded in the committed fixtures in tests/golden/ by
+tests/golden/make_golden.py.
 
 PARITY STATUS: the reference repo holds no golden vectors / known-answer tests for this path
 (SURVEY.md section 4), so the pin is "outputs of the reference itself run here".  Two

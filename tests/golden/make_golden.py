@@ -1,5 +1,5 @@
-"""Generate the committed fixtures from the REFERENCE ITSELF (run in the build container, where
-/root/reference exists):  python tests/golden/make_golden.py
+"""Generate the committed fixtures from the REFERENCE ITSELF (run where a checkout of the reference
+exists, see oracle/ref_loader.py):  python tests/golden/make_golden.py
 
 Weights are not stored (8 MB): they are the PyTorch default init under torch.manual_seed(seed),
 which the reference modules and the engine's parameter containers reproduce identically
@@ -15,6 +15,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from lookoncetohear_b200 import synth  # noqa: E402
+from oracle import golden  # noqa: E402
 from oracle import ref_loader as rl  # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -62,7 +63,64 @@ def main():
             "embed": {k: list(v.shape) for k, v in en.state_dict().items()}}
     with open(os.path.join(HERE, "ckpt_keys.json"), "w") as f:
         json.dump(keys, f, indent=0, sort_keys=True)
+    reference_pins()
     print("written", os.listdir(HERE))
+
+
+def reference_pins():
+    """ref_pins.npz: what tests/test_oracle.py and tests/test_ckpt.py compare with the reference, recorded from it.
+    Tensors too large to store whole are pinned by a sample and their norm (oracle/golden.py)."""
+    import importlib
+    p = {}
+    # seeded default init of both networks (test_seeded_init_matches_reference, the checkpoint tests)
+    for seed in (0, 11, 13):
+        p.update(golden.fingerprint(f"init_sep_{seed}", rl.reference_net(seed).state_dict()))
+    p.update(golden.fingerprint("init_embed_12", rl.reference_embed_net(12).state_dict()))
+    # parameters: names and sizes (test_param_counts)
+    for name, mod in (("sep", rl.reference_net(0)), ("embed", rl.reference_embed_net(0))):
+        params = list(mod.named_parameters())
+        p[f"params_{name}.names"] = np.array([k for k, _ in params])
+        p[f"params_{name}.numel"] = np.array([v.numel() for _, v in params], dtype=np.int64)
+    # whole-utterance output and the final streaming state (test_restatement_equals_reference_forward_and_state)
+    net = rl.reference_net(3)
+    x, _ = synth.mixture(2, 128 * 9 + 77, seed0=50)
+    e = synth.embedding(2, seed0=60)
+    with torch.no_grad():
+        y = net(x, e)
+        st = net.init_buffers(2, "cpu")
+        _, st = net.predict(x, e[:, 0], st)
+    p["fwd_state.wsum"] = weight_checksum(net.state_dict())
+    p["fwd_state.y"] = y.numpy()
+    for k in ("conv_buf", "deconv_buf", "istft_buf"):
+        p.update(golden.pin(f"fwd_state.{k}", st[k]))
+    for i in range(3):
+        for k in ("K_buf", "V_buf", "h0", "c0"):
+            p.update(golden.pin(f"fwd_state.buf{i}.{k}", st["gridnet_bufs"][f"buf{i}"][k]))
+    # fp32 reference output the fp64 restatement is held to (test_restatement_fp64_floor)
+    net = rl.reference_net(1)
+    x, _ = synth.mixture(1, 128 * 8)
+    e = synth.embedding(1)
+    with torch.no_grad():
+        p["fp64_floor.y"] = net(x, e).numpy()
+    p["fp64_floor.wsum"] = weight_checksum(net.state_dict())
+    # enrollment network (test_embed_restatement_equals_reference)
+    en = rl.reference_embed_net(2)
+    with torch.no_grad():
+        p["embed.emb"] = en(synth.enrollment(2, 5000)).numpy()
+    p["embed.wsum"] = weight_checksum(en.state_dict())
+    # the STFT the reference vendors (test_stft_shim_equals_the_stft_the_reference_vendors)
+    stft = importlib.import_module("src.models.tfgridnet_orig.stft").Stft
+    for j, (n_fft, hop, n) in enumerate(((128, 64, 5000), (128, 64, 4999), (192, 128, 3001))):
+        x = synth.enrollment(3, n).transpose(1, 2).contiguous()
+        out, olens = stft(n_fft=n_fft, win_length=n_fft, hop_length=hop, window="hann")(x, torch.tensor([n, n, n]))
+        p.update(golden.pin(f"stft{j}", out, n=1024))
+        p[f"stft{j}.olens"] = olens.numpy()
+    # separator output behind a checkpoint written from the reference (test_checkpoint_outputs_on_gpu)
+    net = rl.reference_net(13)
+    x, _ = synth.mixture(1, 128 * 12)
+    with torch.no_grad():
+        p["ckpt_gpu.y"] = net(x, synth.embedding(1)).numpy()
+    np.savez_compressed(os.path.join(HERE, "ref_pins.npz"), **p)
 
 
 if __name__ == "__main__":

@@ -1,26 +1,31 @@
 """SURVEY section 8(f1): a Lightning checkpoint of the reference loads UNCHANGED into the engine's classes.
 
 The evaluation driver does ``torch.load(run_dir/best.ckpt)['state_dict']`` and ``load_state_dict`` on a
-LightningModule whose ``self.model`` is the network (/root/reference/src/ts_hear_test.py:18-34,
+LightningModule whose ``self.model`` is the network (the reference's src/ts_hear_test.py:18-34,
 ts_hear_embed_pl_module.py:25), so every key carries a ``model.`` prefix; real asteroid registers one extra buffer
-per filterbank (``torch_window``).  Where the reference checkout exists the checkpoint is written from the
-reference's own modules; everywhere, the key names and shapes are pinned by a committed fixture generated from
-the reference (tests/golden/make_golden.py -> ckpt_keys.json).
+per filterbank (``torch_window``).  The checkpoints hold the state_dict of a seeded reference module: key names and
+shapes as recorded from the reference (ckpt_keys.json), values as the seeded init reproduces them, checked against
+the reference's own per-key fingerprint (ref_pins.npz; both written by tests/golden/make_golden.py).
 """
 import json
 import os
 
+import numpy as np
 import pytest
 import torch
 import torch.nn as nn
 
 from lookoncetohear_b200 import EmbedTFGridNet, Net, synth
 from lookoncetohear_b200.net import SepState
-from oracle import ref_loader as rl
+from oracle import golden
 from oracle import restate as rs
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-needs_ref = pytest.mark.skipif(not rl.available(), reason="reference checkout not present on this box")
+
+
+@pytest.fixture(scope="module")
+def pins():
+    return np.load(os.path.join(GOLD, "ref_pins.npz"))
 
 
 class _PLShaped(nn.Module):
@@ -31,16 +36,25 @@ class _PLShaped(nn.Module):
         self.model = model
 
 
-def _write_ckpt(path, module, extra=None):
-    sd = {k: v.detach().clone() for k, v in _PLShaped(module).state_dict().items()}
+def _reference_state_dict(pins, name, seed, module):
+    """The state_dict of the reference's `name` ('sep' / 'embed') network built under torch.manual_seed(seed)."""
+    torch.manual_seed(seed)
+    sd = {k: v.detach().clone() for k, v in module().state_dict().items()}
+    with open(os.path.join(GOLD, "ckpt_keys.json")) as f:
+        assert {k: list(v.shape) for k, v in sd.items()} == json.load(f)[name]
+    assert golden.fingerprint_mismatches(pins, f"init_{name}_{seed}", sd) == []
+    return sd
+
+
+def _write_ckpt(path, net_sd, extra=None):
+    sd = {"model." + k: v for k, v in net_sd.items()}                 # _PLShaped(network).state_dict()
     sd.update(extra or {})
     torch.save({"state_dict": sd, "epoch": 7, "global_step": 1234}, path)
     return sd
 
 
-@needs_ref
-def test_separator_checkpoint_loads_strict(tmp_path, tsh_params):
-    ref = rl.reference_net(11)
+def test_separator_checkpoint_loads_strict(tmp_path, tsh_params, pins):
+    ref = _reference_state_dict(pins, "sep", 11, lambda: Net(**tsh_params))
     path = os.path.join(tmp_path, "best.ckpt")
     extra = {"model.tfgridnet.enc.filterbank.torch_window": torch.hann_window(192),
              "model.tfgridnet.dec.filterbank.torch_window": torch.hann_window(192)}
@@ -56,9 +70,8 @@ def test_separator_checkpoint_loads_strict(tmp_path, tsh_params):
     assert mine.model._dirty                                # the engine repacks on the next call
 
 
-@needs_ref
-def test_enrollment_checkpoint_loads_strict(tmp_path, embed_params):
-    ref = rl.reference_embed_net(12)
+def test_enrollment_checkpoint_loads_strict(tmp_path, embed_params, pins):
+    ref = _reference_state_dict(pins, "embed", 12, lambda: EmbedTFGridNet(**embed_params))
     path = os.path.join(tmp_path, "embed.ckpt")
     sd = _write_ckpt(path, ref)
     torch.manual_seed(98)
@@ -109,9 +122,8 @@ def test_net_deepcopy_and_pickle(tsh_params):
 
 
 @pytest.mark.gpu
-@needs_ref
-def test_checkpoint_outputs_on_gpu(tmp_path, tsh_params):
-    ref = rl.reference_net(13)
+def test_checkpoint_outputs_on_gpu(tmp_path, tsh_params, pins):
+    ref = _reference_state_dict(pins, "sep", 13, lambda: Net(**tsh_params))
     path = os.path.join(tmp_path, "best.ckpt")
     _write_ckpt(path, ref)
     mine = _PLShaped(Net(**tsh_params))
@@ -121,8 +133,7 @@ def test_checkpoint_outputs_on_gpu(tmp_path, tsh_params):
     e = synth.embedding(1)
     with torch.no_grad():
         y = mine.model(x.cuda(), e.cuda()).cpu()
-        y_ref = ref(x, e)
-    assert rs.rel_l2(y, y_ref) <= 1e-3
+    assert rs.rel_l2(y, torch.from_numpy(pins["ckpt_gpu.y"])) <= 1e-3
 
 
 @pytest.mark.gpu

@@ -1,6 +1,7 @@
-"""Pin the oracle (oracle/restate.py): against the reference's own code where the checkout exists
-(build container), and against the committed fixtures generated from the reference (everywhere).
-The reference repo has no golden vectors of its own (SURVEY.md section 4)."""
+"""Pin the oracle (oracle/restate.py) against the reference: every comparison is with results of the
+reference's own code, recorded in the committed fixtures by tests/golden/make_golden.py (ref_pins.npz
+holds the large ones as samples plus norms, oracle/golden.py).  The reference repo has no golden
+vectors of its own (SURVEY.md section 4)."""
 import os
 
 import numpy as np
@@ -8,12 +9,17 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from lookoncetohear_b200 import Net, synth
-from oracle import ref_loader as rl
+from lookoncetohear_b200 import EmbedTFGridNet, Net, synth
+from oracle import golden
 from oracle import restate as rs
 
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-needs_ref = pytest.mark.skipif(not rl.available(), reason="reference checkout not present on this box")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLD = os.path.join(ROOT, "tests", "golden")
+
+
+@pytest.fixture(scope="module")
+def pins():
+    return np.load(os.path.join(GOLD, "ref_pins.npz"))
 
 
 def _wsum(sd):
@@ -26,61 +32,48 @@ def _seeded_sd(tsh_params, seed):
     return {k: v.detach().clone() for k, v in Net(**tsh_params).state_dict().items()}
 
 
-@needs_ref
-def test_seeded_init_matches_reference(tsh_params):
-    ref = rl.reference_net(0).state_dict()
-    mine = _seeded_sd(tsh_params, 0)
-    assert set(ref) == set(mine)
-    for k in ref:
-        assert torch.allclose(ref[k], mine[k], atol=1e-7, rtol=0), k
+def test_seeded_init_matches_reference(tsh_params, pins):
+    """The engine's parameter containers under a seed hold the reference's seeded default init."""
+    assert golden.fingerprint_mismatches(pins, "init_sep_0", _seeded_sd(tsh_params, 0), atol=1e-7) == []
 
 
-@needs_ref
-def test_param_counts():
-    assert sum(p.numel() for p in rl.reference_net(0).parameters()) == 2_037_960
-    assert sum(p.numel() for p in rl.reference_embed_net(0).parameters()) == 2_368_681
+def test_param_counts(pins, tsh_params, embed_params):
+    for name, total, mod in (("sep", 2_037_960, Net(**tsh_params)), ("embed", 2_368_681, EmbedTFGridNet(**embed_params))):
+        ref = dict(zip(pins[f"params_{name}.names"].tolist(), pins[f"params_{name}.numel"].tolist()))
+        assert sum(ref.values()) == total, name
+        assert {k: p.numel() for k, p in mod.named_parameters()} == ref, name
 
 
-@needs_ref
-def test_restatement_equals_reference_forward_and_state():
-    net = rl.reference_net(3)
-    sd = {k: v.clone() for k, v in net.state_dict().items()}
+def test_restatement_equals_reference_forward_and_state(tsh_params, pins):
+    sd = _seeded_sd(tsh_params, 3)
+    assert np.allclose(_wsum(sd), pins["fwd_state.wsum"], rtol=1e-9), "seeded init differs from the build that made the fixture"
     x, _ = synth.mixture(2, 128 * 9 + 77, seed0=50)
     e = synth.embedding(2, seed0=60)
-    with torch.no_grad():
-        y_ref = net(x, e)
-        st_ref = net.init_buffers(2, "cpu")
-        _, st_ref = net.predict(x, e[:, 0], st_ref)
     st = rs.sep_init_state(sd, 2)
     y, st = rs.sep_predict(sd, x, e[:, 0], st)
-    assert rs.rel_l2(y, y_ref) < 5e-6
+    assert rs.rel_l2(y, torch.from_numpy(pins["fwd_state.y"])) < 5e-6
     for k in ("conv_buf", "deconv_buf", "istft_buf"):
-        assert rs.rel_l2(st[k], st_ref[k]) < 5e-6, k
+        assert golden.pin_error(pins, f"fwd_state.{k}", st[k]) < 5e-6, k
     for i in range(3):
         for k in ("K_buf", "V_buf", "h0", "c0"):
-            assert rs.rel_l2(st["gridnet_bufs"][f"buf{i}"][k], st_ref["gridnet_bufs"][f"buf{i}"][k]) < 5e-6
+            assert golden.pin_error(pins, f"fwd_state.buf{i}.{k}", st["gridnet_bufs"][f"buf{i}"][k]) < 5e-6, (i, k)
 
 
-@needs_ref
-def test_restatement_fp64_floor():
-    net = rl.reference_net(1)
-    sd = {k: v.clone() for k, v in net.state_dict().items()}
+def test_restatement_fp64_floor(tsh_params, pins):
+    sd = _seeded_sd(tsh_params, 1)
+    assert np.allclose(_wsum(sd), pins["fp64_floor.wsum"], rtol=1e-9), "seeded init differs from the build that made the fixture"
     x, _ = synth.mixture(1, 128 * 8)
     e = synth.embedding(1)
-    with torch.no_grad():
-        y_ref = net(x, e)
     y64 = rs.sep_forward(rs.cast_sd(sd, torch.float64), x.double(), e.double())
-    assert rs.rel_l2(y64, y_ref) < 5e-6
+    assert rs.rel_l2(y64, torch.from_numpy(pins["fp64_floor.y"])) < 5e-6
 
 
-@needs_ref
-def test_embed_restatement_equals_reference():
-    en = rl.reference_embed_net(2)
-    sd = {k: v.clone() for k, v in en.state_dict().items()}
-    x = synth.enrollment(2, 5000)
-    with torch.no_grad():
-        r = en(x)
-    o = rs.embed_forward(sd, x)
+def test_embed_restatement_equals_reference(embed_params, pins):
+    torch.manual_seed(2)
+    sd = {k: v.detach().clone() for k, v in EmbedTFGridNet(**embed_params).state_dict().items()}
+    assert np.allclose(_wsum(sd), pins["embed.wsum"], rtol=1e-9), "seeded init differs from the build that made the fixture"
+    o = rs.embed_forward(sd, synth.enrollment(2, 5000))
+    r = torch.from_numpy(pins["embed.emb"])
     assert rs.rel_l2(o, r) < 5e-5
     assert float(F.cosine_similarity(o, r).min()) > 0.99999
 
@@ -141,20 +134,17 @@ def test_si_sdr_known_answer():
     assert abs(float(rs.si_sdr(p, t)) - 20 * np.log10(1 / 0.3)) < 1e-3
 
 
-@needs_ref
-def test_stft_shim_equals_the_stft_the_reference_vendors():
+def test_stft_shim_equals_the_stft_the_reference_vendors(pins, monkeypatch):
     """The one piece of espnet2 arithmetic the reference DOES carry -- Stft.forward, src/models/tfgridnet_orig/
     stft.py:68-195, identical to what espnet2's STFTEncoder calls -- pins the shim the enrollment oracle uses
     (oracle/shims/espnet2/enh/encoder/stft_encoder.py): same frames, same bins, same values, same output lengths."""
-    import importlib
-    rl._prepare()
-    vendored = importlib.import_module("src.models.tfgridnet_orig.stft").Stft
+    monkeypatch.syspath_prepend(os.path.join(ROOT, "oracle", "shims"))
     from espnet2.enh.encoder.stft_encoder import STFTEncoder
-    for n_fft, hop, n in ((128, 64, 5000), (128, 64, 4999), (192, 128, 3001)):
+    for j, (n_fft, hop, n) in enumerate(((128, 64, 5000), (128, 64, 4999), (192, 128, 3001))):
         x = synth.enrollment(3, n).transpose(1, 2).contiguous()          # [B, N, M] as EmbedTFGridNet.forward passes it
         ilens = torch.tensor([n, n, n])
-        ref, rl_out = vendored(n_fft=n_fft, win_length=n_fft, hop_length=hop, window="hann")(x, ilens)     # [B,T,M,F,2]
         got, gl_out = STFTEncoder(n_fft, n_fft, hop, window="hann")(x, ilens)                             # complex [B,T,M,F]
-        assert got.shape == ref.shape[:-1] and got.shape[1] == 1 + n // hop
-        assert torch.equal(rl_out, gl_out)
-        assert rs.rel_l2(torch.view_as_real(got), ref) < 1e-6
+        ref_shape = tuple(pins[f"stft{j}.shape"])                                                          # [B,T,M,F,2]
+        assert got.shape == ref_shape[:-1] and got.shape[1] == 1 + n // hop
+        assert gl_out.tolist() == pins[f"stft{j}.olens"].tolist()
+        assert golden.pin_error(pins, f"stft{j}", torch.view_as_real(got)) < 1e-6
