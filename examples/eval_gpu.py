@@ -5,9 +5,10 @@
     enrollment recording --EmbedTFGridNet--> embedding                             (ts_hear_test.py:133-135)
     model(mixture, embedding) --Net--> outputs                                     (ts_hear_test.py:138)
     eval_metrics(outputs, target, mixture, embedding, embedding_gt)                (ts_hear_test.py:139-146)
+    binaural_errors(outputs, target, sr, moving)  ILD / ITD errors                  (src/eval/binaural.py:49-149)
 
 Synthetic inputs (no dataset in the image): white-noise events, exponentially decaying random impulse responses.  Only the
-three metric floats per mixture leave the device.  Usage: python examples/eval_gpu.py [n_batches] [batch]"""
+metric floats per mixture leave the device.  Usage: python examples/eval_gpu.py [n_batches] [batch]"""
 import os
 import sys
 import time
@@ -17,7 +18,7 @@ import torch
 
 from lookoncetohear_b200 import EmbedTFGridNet, Net
 from lookoncetohear_b200.configs import EMBED_PARAMS, TSH_PARAMS
-from lookoncetohear_b200.metrics import eval_metrics
+from lookoncetohear_b200.metrics import binaural_errors, eval_metrics
 from lookoncetohear_b200.render import render_binaural
 
 
@@ -51,10 +52,12 @@ def main():
             embedding = enroll_model(enrollment).unsqueeze(1)                  # [B, 1, 256]
             embedding_gt = torch.nn.functional.normalize(torch.rand(batch, 1, 256, generator=gen, device=dev), dim=-1)
             outputs = model(mixture, embedding)
-            rows.append(eval_metrics(outputs, target, mixture, embedding, embedding_gt))
+            rows.append(torch.cat([eval_metrics(outputs, target, mixture, embedding, embedding_gt),
+                                   binaural_errors(outputs, target, 16000),                 # static, whole 5 s
+                                   binaural_errors(outputs, target, 16000, moving=True)], 1))   # 250 ms windows
     res = torch.cat(rows).cpu()                                                # the only device -> host copy
     dt = time.perf_counter() - t0
-    print("output_sisnr  si_snr_i  embedding_sim")
+    print("output_sisnr  si_snr_i  embedding_sim  ild_diff_dB  itd_diff_us  ild_diff_moving  itd_diff_moving")
     print(res)
     print(f"{res.shape[0]} mixtures of 5 s in {dt:.2f} s wall (first call includes weight upload); Average SI-SNRi {res[:, 1].mean():.3f}")
 

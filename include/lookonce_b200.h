@@ -236,6 +236,29 @@ int l2h_render_binaural(const float* src_dev, const float* rir_dev, const float*
                         int32_t batch, int32_t n_src, int32_t n_samples, int32_t rir_len, float* events_dev,
                         float* mixture_dev, float* norm_dev, void* scratch_dev, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Binaural cue errors on the device (src/eval/binaural.py:6-149): per mixture b,
+ * out_dev[b] = { ild_diff (dB), itd_diff (microseconds) } of est against gt, both [batch][2][n_samples] fp32 contiguous,
+ * ear 0 = left.  Windows of `frame` samples, the last zero-padded past n_samples (chunk_and_mask :6-42); frame = 0 is one
+ * window of the whole signal (the static form).  Per window:
+ *   ILD = 10 log10(sum left^2 / sum right^2)                                                    compute_ild :44-47
+ *   ITD = tau / sr * 1e6, tau = first argmax over k in [-t, t] of |sum_n left[(n+k) mod L] right[n]|,
+ *         t = min(t_max, L/2), L = the window length                          axiswise_xcorr :83-92, compute_itd :94-117
+ *   valid = max over ears of sqrt(mean(gt^2)) >= rms_threshold (frame > 0 only; every static window is valid)
+ * Per mixture: ild_diff = |mean_valid ild_est - mean_valid ild_gt|, itd_diff = mean_valid |itd_est - itd_gt|
+ * (ild_diff :62-81, itd_diff :134-147; with one window these are the static |differences|).  Non-finite results are
+ * the reference's: a silent ear gives +-inf or NaN ILD, a mixture without a valid window NaN.
+ * The caller passes the reference's integers: frame = round(0.25 sr), t_max = round(1e-3 sr) (Python rounding).
+ * t_max = 0 computes ILD only (itd entries are NaN).  Refused: t_max > 256, and t_max > 0 with an odd window length
+ * (the reference's irfft drops a sample there, its "correlation" is not one).
+ * windows_dev [batch][n_windows][5] = { ild_est, ild_gt, itd_est, itd_gt, valid (0/1) } or NULL,
+ * n_windows = frame ? 1 + (n_samples - 1) / frame : 1.  workspace_dev: l2h_eval_binaural_workspace_bytes() bytes on the
+ * device.  Asynchronous on `stream`, no allocation, no host synchronisation; fixed-order sums (bit-reproducible). */
+int l2h_eval_binaural_workspace_bytes(int32_t batch, int32_t n_samples, int32_t frame, int32_t t_max, size_t* bytes);
+int l2h_eval_binaural(const float* est_dev, const float* gt_dev, int32_t batch, int32_t n_samples, int32_t frame,
+                      int32_t t_max, double rms_threshold, int32_t sr, float* out_dev, float* windows_dev,
+                      void* workspace_dev, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

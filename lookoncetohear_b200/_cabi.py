@@ -78,6 +78,11 @@ _SIGS = {
     "l2h_eval_metrics": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32,
                                        ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p,
                                        ctypes.c_void_p]),
+    "l2h_eval_binaural_workspace_bytes": (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
+                                                        ctypes.POINTER(ctypes.c_size_t)]),
+    "l2h_eval_binaural": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
+                                        ctypes.c_int32, ctypes.c_double, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p,
+                                        ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]),
     "l2h_render_binaural": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32,
                                           ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p,
                                           ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),

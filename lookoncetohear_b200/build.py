@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "liblookonce_b200.so")
-SOURCES = ["sep_engine.cu", "embed_engine.cu", "umma_gemm.cu", "eval_metrics.cu", "render.cu"]
+SOURCES = ["sep_engine.cu", "embed_engine.cu", "umma_gemm.cu", "eval_metrics.cu", "render.cu", "binaural_metrics.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "--compiler-options", "-fPIC", "-shared", "-Xptxas", "-v"]
 
